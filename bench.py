@@ -18,7 +18,10 @@ reference encoder (oracle/_ref) run on the same picture order: "parity_checked" 
 mismatch fails the run.  A second workload point ("workload_hard": +-8 noise, few skipped macroblocks, ~27x the bits) is reported
 next to the headline.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--streams S] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--streams S] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the headline (resident) path handed back in its last timed step as DIR/*.npy (see
+dump_outputs); the pictures are the same from run to run, so two builds can be compared output for output.
 
 N > 1: one process per GPU under torch.distributed (launched by the driver with torchrun); streams are
 independent, there is no data-path collective ("scaling": "weak"); NCCL is used only for the barrier and the
@@ -332,7 +335,7 @@ def decode_bench(local, clip, seq, peak, S=256, n_pictures=8):
 
 def api_run(args, local, clip_path, out_prefix, S):
     """S threads x S ISVCEncoder objects through libopenh264_b200_wels.so (the reference's API), timed inside the driver"""
-    drv = os.path.join(ROOT, "oracle", "_ref", "wels_mt_driver")
+    drv = os.path.join(ROOT, "tests", "wels", "build", "wels_mt_driver")
     lib = os.path.join(ROOT, "openh264_b200", "libopenh264_b200_wels.so")
     if not (os.path.exists(drv) and os.path.exists(lib)):
         return None
@@ -349,6 +352,25 @@ def api_run(args, local, clip_path, out_prefix, S):
     return res
 
 
+def dump_outputs(out_dir, aus, frame_types, limit=64_000_000):
+    """The access units of one step (one per stream) and their frame types, as float arrays: bitstream.npy = the bytes of the
+    dumped streams' access units one after the other, au_bytes.npy = their lengths, streams.npy = the stream indices,
+    frame_type.npy = EVideoFrameType per dumped stream.  Streams are taken in a fixed seeded order while their bytes fit
+    into `limit` as float32 (at 1080p a step of 256 streams is larger than that)."""
+    os.makedirs(out_dir, exist_ok=True)
+    pick, total = [], 0
+    for s in np.random.RandomState(264).permutation(len(aus)):
+        if total + 4 * len(aus[s]) > limit - 1_000_000:        # 1 MB left for the small arrays
+            break
+        pick.append(int(s))
+        total += 4 * len(aus[s])
+    pick.sort()
+    np.save(os.path.join(out_dir, "bitstream.npy"), np.frombuffer(b"".join(aus[s] for s in pick), np.uint8).astype(np.float32))
+    np.save(os.path.join(out_dir, "au_bytes.npy"), np.array([len(aus[s]) for s in pick], np.float64))
+    np.save(os.path.join(out_dir, "streams.npy"), np.array(pick, np.float64))
+    np.save(os.path.join(out_dir, "frame_type.npy"), np.array([frame_types[s] for s in pick], np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -363,6 +385,7 @@ def main():
     ap.add_argument("--no-api", action="store_true", help="skip the run through ISVCEncoder::EncodeFrame")
     ap.add_argument("--no-decode", action="store_true", help="skip the decoder throughput block")
     ap.add_argument("--no-parity", action="store_true", help="skip the reference comparison of the produced bitstreams")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the access units of the last timed step as DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
@@ -399,20 +422,22 @@ def main():
     def timed_run(enc, on_dev, warmup, steps, keep, **kw):
         """pipelined submit/collect (two batches in flight); returns timing + per-stream access units (if keep)"""
         aus = [[] for _ in range(S)] if keep else None
+        last = None
         kern, d2h, coded_mbs = [], [], []
         nb = 0
 
         def loop(first, count, timed):
-            nonlocal nb
+            nonlocal nb, last
             enc.submit(srcs(first, on_dev, **kw), on_device=on_dev)
             for i in range(1, count + 1):
                 if i < count:
                     enc.submit(srcs(first + i, on_dev, **kw), on_device=on_dev)
-                bs, _ = enc.collect()
+                bs, ft = enc.collect()
                 if keep:
                     for s in range(S):
                         aus[s].append(bs[s])
                 if timed:
+                    last = (bs, ft)
                     nb += sum(len(b) for b in bs)
                     kern.append(enc.timing_us())
                     d2h.append(enc.d2h_bytes())
@@ -437,7 +462,7 @@ def main():
         sampler.join(timeout=2)
         dt, pics = shard.job_totals(max(wall, dev), S * steps, device="cuda")   # MAX over ranks / SUM over ranks
         return {"dt": dt, "pictures": pics, "wall": wall, "dev": dev, "bytes": nb, "clocks": sampler.summary(), "kern": kern, "d2h": d2h,
-                "coded": coded_mbs, "aus": aus}
+                "coded": coded_mbs, "aus": aus, "last": last}
 
     results = {}
     launches0 = L.b2h264_launch_count()
@@ -510,6 +535,9 @@ def main():
         hard = {"generator": "same synthetic generator, +-%d per-frame noise" % HARD_NOISE, "value": r["pictures"] / r["dt"], "unit": "frames/s",
                 "steps": hsteps, "skip_ratio": 1.0 - coded / (S * MBS_PER_FRAME), "bitstream_kbytes_per_frame": r["bytes"] / (S * hsteps) / 1e3,
                 "encode_kernel_ms": float(np.mean([k[0] for k in r["kern"]])) * 1e-3, "host_entropy_ms": float(np.mean([k[2] for k in r["kern"]])) * 1e-3}
+
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, *results["resident"]["last"])
 
     if rank == 0:
         res, l2 = results["resident"], results["e2e_layer2"]

@@ -17,7 +17,7 @@
 
 #include "b2h264_codec.h"
 #include "broker.h"
-#include "codec_api.h"
+#include "b2h264_wels_abi.h"
 
 namespace {
 

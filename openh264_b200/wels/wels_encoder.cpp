@@ -1,8 +1,8 @@
 // wels_encoder.cpp — layer 3: an ISVCEncoder (codec/api/wels/codec_api.h:272-339) over the layer-2 C ABI
 // (include/b2h264_codec.h).  One object = one stream, but NOT one private GPU encoder: objects of equal configuration
-// are streams of a shared batched encoder and their EncodeFrame calls are coded together (broker.h).  Compiled against the reference's public API headers so that
-// the vtable slot order and the parameter / bitstream-info structures are the reference's own
-// (include/b2h264_wels_api.h).  Behavioural model: CWelsH264SVCEncoder (codec/encoder/plus/src/welsEncoderExt.cpp):
+// are streams of a shared batched encoder and their EncodeFrame calls are coded together (broker.h).  The vtable slot
+// order and the parameter / bitstream-info structures are the reference's own (include/b2h264_wels_abi.h,
+// include/b2h264_wels_api.h).  Behavioural model: CWelsH264SVCEncoder (codec/encoder/plus/src/welsEncoderExt.cpp):
 // Initialize* validate and (re)create the encoder, EncodeFrame is synchronous and returns encoder-owned bitstream
 // memory that stays valid until the next call.  No CPU encoder lives here: every picture goes through
 // b2h264_enc_submit / b2h264_enc_collect, i.e. the CUDA macroblock pipeline; creation fails without a device.
@@ -14,8 +14,7 @@
 
 #include "b2h264_codec.h"
 #include "broker.h"
-#include "codec_api.h"
-#include "codec_ver.h"
+#include "b2h264_wels_abi.h"
 
 namespace {
 

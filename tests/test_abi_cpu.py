@@ -34,7 +34,7 @@ def test_every_declared_symbol_is_exported(L):
     # include/b2h264_wels_api.h) in libopenh264_b200_wels.so, which links against the former
     import ctypes
     wels_so = os.path.join(ROOT, "openh264_b200", "libopenh264_b200_wels.so")
-    assert os.path.exists(wels_so), "build() makes it where the reference's public headers exist; it ships prebuilt"
+    assert os.path.exists(wels_so), "build() makes it"
     Wl = ctypes.CDLL(wels_so)
     missing = [n for n in declared_symbols() if not hasattr(Wl if n.startswith("Wels") else L, n)]
     assert not missing, missing

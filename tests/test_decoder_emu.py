@@ -2,9 +2,11 @@
 openh264_b200/csrc/dec_mb.cuh (prediction + dequant + inverse transform + reconstruction from parsed macroblock
 records, then the same deblocking code the encoder path uses) behind the host bitstream parser
 (openh264_b200/csrc/h264_parse.cpp) must reproduce the reference decoder's pictures bit for bit
-(ISVCDecoder::DecodeFrameNoDelay through oracle/_ref) on streams the REFERENCE ENCODER produced.
+(ISVCDecoder::DecodeFrameNoDelay through oracle/_ref, or its stored picture hashes) on streams the REFERENCE ENCODER produced.
 The device kernel that batches this stage does not exist yet; the product decoder entry points still fail loudly."""
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 import sys
@@ -23,6 +25,8 @@ def emu():
     E = C.CDLL(os.path.join(ROOT, "tests", "emu", "libb2h264_emu.so"))
     E.emu_decode.restype = C.c_int
     E.emu_decode.argtypes = [C.c_void_p, C.c_long, C.c_void_p, C.c_long, C.POINTER(C.c_int), C.POINTER(C.c_int)]
+    E.emu_encode.restype = C.c_long
+    E.emu_encode.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p, C.c_long, C.c_void_p, C.c_void_p]
     return E
 
 
@@ -40,18 +44,21 @@ CASES = [(176, 144, 6, 26, 1), (176, 144, 5, 0, 2), (176, 144, 5, 51, 2), (320, 
          (16, 16, 4, 26, 5), (640, 360, 4, 34, 6), (64, 256, 4, 18, 7)]
 
 
-@pytest.mark.parametrize("case", CASES)
-def test_host_decoder_matches_reference_decoder(emu, case):
-    if not h264lib.have_ref():
-        pytest.skip("reference build not on this machine")
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    from make_encoder_golden import ref_encode
-    w, h, n, qp, seed = case
-    yuv = h264lib.synth_clip(w, h, n, seed=seed)
-    bs, _, _ = ref_encode(yuv, w, h, n, qp, 30.0)                      # stream from the REFERENCE encoder
-    bs = bytes(bs)
-    nr, rw, rh, want = ref_decode(bs)
-    assert nr == n and (rw, rh) == (w, h)
+DEC_GOLD = json.load(open(os.path.join(ROOT, "tests", "golden", "decoder_emu.json")))
+RES = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_res.json")))["h264dec"]
+
+
+def reference_stream(emu, key, yuv, w, h, n, qp, fps):
+    """the reference encoder's stream of `yuv` and the SHA-1 of every picture the reference decoder makes of it
+    (tests/golden/make_decoder_emu_golden.py).  The stream is rebuilt by the host build of the encoder, which reproduces
+    the reference encoder bit for bit (tests/test_encoder_emu.py); its SHA-1 is checked against the reference's."""
+    from test_encoder_emu import emu_encode
+    bs, _ = emu_encode(emu, yuv, w, h, n, qp, fps)
+    assert hashlib.sha1(bs).hexdigest() == DEC_GOLD[key]["stream_sha1"]
+    return bs, DEC_GOLD[key]["pictures"]
+
+
+def decode_and_check(emu, bs, w, h, n, want):
     a = np.frombuffer(bs, np.uint8)
     out = np.zeros(n * w * h * 3 // 2 + 64, np.uint8)
     W, H = C.c_int(), C.c_int()
@@ -60,48 +67,51 @@ def test_host_decoder_matches_reference_decoder(emu, case):
     assert (W.value, H.value) == (w, h)
     fsz = w * h * 3 // 2
     for f in range(n):
-        assert np.array_equal(out[f * fsz:(f + 1) * fsz], want[f * fsz:(f + 1) * fsz]), "picture %d differs" % f
+        assert hashlib.sha1(out[f * fsz:(f + 1) * fsz].tobytes()).hexdigest() == want[f], "picture %d differs" % f
+
+
+def case_key(case):
+    return "%dx%d_n%d_qp%d_s%d" % case
+
+
+@pytest.mark.parametrize("case", CASES)
+def test_host_decoder_matches_reference_decoder(emu, case):
+    w, h, n, qp, seed = case
+    bs, want = reference_stream(emu, case_key(case), h264lib.synth_clip(w, h, n, seed=seed), w, h, n, qp, 30.0)
+    assert len(want) == n
+    decode_and_check(emu, bs, w, h, n, want)
+
+
+OWN_CLIP = os.path.join(ROOT, "tests", "golden", "CiscoVT2people_320x192_12fps.yuv")
 
 
 def test_host_decoder_on_the_references_own_clip(emu):
-    clip = "/root/reference/res/CiscoVT2people_320x192_12fps.yuv"
-    if not (h264lib.have_ref() and os.path.exists(clip)):
-        pytest.skip("reference build / clip not on this machine")
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    from make_encoder_golden import ref_encode
-    yuv = np.fromfile(clip, dtype=np.uint8)
-    bs = bytes(ref_encode(yuv, 320, 192, 9, 28, 12.0)[0])
-    nr, rw, rh, want = ref_decode(bs)
-    a = np.frombuffer(bs, np.uint8)
-    out = np.zeros(want.size + 64, np.uint8)
-    W, H = C.c_int(), C.c_int()
-    assert emu.emu_decode(a.ctypes.data, len(a), out.ctypes.data, out.size, C.byref(W), C.byref(H)) == nr == 9
-    assert np.array_equal(out[:want.size], want)
+    yuv = np.fromfile(OWN_CLIP, dtype=np.uint8)
+    bs, want = reference_stream(emu, "own_clip_320x192_n9_qp28", yuv, 320, 192, 9, 28, 12.0)
+    decode_and_check(emu, bs, 320, 192, 9, want)
 
 
 def test_unsupported_streams_are_rejected_not_guessed(emu):
     """a stream with scaling lists (outside the supported class) must come back as a parse error, never as pictures"""
-    path = "/root/reference/res/test_scalinglist_jm.264"
-    if not os.path.exists(path):
-        pytest.skip("reference bitstreams not on this machine")
-    a = np.fromfile(path, dtype=np.uint8)
+    a = np.fromfile(os.path.join(ROOT, "tests", "golden", "reference_res", "test_scalinglist_jm.264"), dtype=np.uint8)
     out = np.zeros(1 << 20, np.uint8)
     W, H = C.c_int(), C.c_int()
     assert emu.emu_decode(a.ctypes.data, len(a), out.ctypes.data, out.size, C.byref(W), C.byref(H)) < 0
 
 
 def test_reference_conformance_table_exact_or_rejected(emu):
-    """every bitstream of the reference's decoder golden table (test/api/decoder_test.cpp) either decodes to the
-    PUBLISHED hash or is rejected as outside the supported stream class — never a wrong picture"""
-    import hashlib
-    import json
+    """every bitstream of the reference's decoder golden table (test/api/decoder_test.cpp) either decodes to what the reference
+    decoder makes of it or is rejected as outside the supported stream class — never a wrong picture.  The streams are the
+    stored ones (tests/golden/reference_res.json): whole streams against their PUBLISHED hash, the first access units of the
+    long ones against the compiled reference's pictures of the same units"""
     tab = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_decoder_hashes.json")))["pairs"]
-    if not os.path.exists("/root/reference/" + tab[0][0]):
-        pytest.skip("reference bitstreams not on this machine")
     out = np.zeros(400 << 20, np.uint8)
     exact, wrong = [], []
     for path, sha in tab:
-        a = np.fromfile("/root/reference/" + path, dtype=np.uint8)
+        stored = RES[os.path.basename(path)]
+        if not stored["whole"]:
+            sha = stored["sha1"]
+        a = np.fromfile(os.path.join(ROOT, "tests", "golden", stored["file"]), dtype=np.uint8)
         W, H = C.c_int(), C.c_int()
         n = emu.emu_decode(a.ctypes.data, len(a), out.ctypes.data, out.size, C.byref(W), C.byref(H))
         if n < 0:

@@ -1,8 +1,8 @@
 """CPU-side check of the encoder's macroblock pipeline SOURCE: the host emulation build (tests/emu, the same
 enc_*.cuh code compiled as a 1-lane warp and run in raster order) must reproduce the reference encoder's
 bitstream bit for bit — against the golden SHA-1s generated from the reference (tests/golden/encoder.json) and,
-where oracle/_ref exists, against the reference run side by side (incl. the reference's own
-res/CiscoVT2people_320x192_12fps.yuv clip, BASELINE.json config 2).  The GPU build of the same source is
+where oracle/_ref exists, against the reference run side by side, and against the reference's bitstreams of its own
+res/*.yuv clips (BASELINE.json config 2 among them; stored samples, tests/golden/make_reference_res_golden.py).  The GPU build of the same source is
 checked by tests/test_gpu_encoder.py."""
 import ctypes as C
 import hashlib
@@ -51,18 +51,22 @@ def test_emu_matches_golden(emu, key):
     assert hashlib.sha1(bs).hexdigest() == GOLD[key]["sha1"]
 
 
+RES_ENCODE = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_res.json")))["encode"]
+
+
+def check_reference_clip(emu, key):
+    """the host build on one of the reference's own clips against the reference encoder's bitstream of it"""
+    g = RES_ENCODE[key]
+    w, h, n = g["w"], g["h"], g["n"]
+    path = os.path.join(ROOT, "tests", "golden", "reference_res", g["clip"])                 # n pictures and the next
+    yuv = np.load(path) if path.endswith(".npy") else np.fromfile(path, dtype=np.uint8)
+    bs, fb = emu_encode(emu, yuv, w, h, n, g["qp"], g["fps"], entropy=tuple(g["entropy"]))
+    assert fb == g["frame_bytes"] and hashlib.sha1(bs).hexdigest() == g["sha1"], key
+
+
 def test_emu_matches_reference_on_its_own_clip(emu):
-    clip = "/root/reference/res/CiscoVT2people_320x192_12fps.yuv"
-    if not (h264lib.have_ref() and os.path.exists(clip)):
-        pytest.skip("reference build / clip not on this machine")
-    import sys
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    from make_encoder_golden import ref_encode
-    yuv = np.fromfile(clip, dtype=np.uint8)
     for qp in (26, 34):
-        ref_bs, ref_fb, _ = ref_encode(yuv, 320, 192, 9, qp, 12.0)
-        bs, fb = emu_encode(emu, yuv, 320, 192, 9, qp, 12.0)
-        assert fb == ref_fb and bs == ref_bs
+        check_reference_clip(emu, "own_clip_qp%d" % qp)
 
 
 EDGE_CASES = [
@@ -91,29 +95,9 @@ def test_emu_matches_reference_edge_cases(emu, case):
 
 
 def test_emu_matches_reference_on_other_reference_clips(emu):
-    """more of the reference's own res/*.yuv clips (first pictures), where they exist"""
-    if not h264lib.have_ref():
-        pytest.skip("reference build not on this machine")
-    import sys
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    from make_encoder_golden import ref_encode
-    clips = [("/root/reference/res/Cisco_Absolute_Power_1280x720_30fps.yuv", 1280, 720, 2, 30),
-             ("/root/reference/res/CiscoVT2people_160x96_6fps.yuv", 160, 96, 6, 24),
-             ("/root/reference/res/Static_152_100.yuv", 152, 100, 8, 28)]
-    ran = 0
-    for path, w, h, n, qp in clips:
-        if not os.path.exists(path):
-            continue
-        fsz = w * h * 3 // 2
-        yuv = np.fromfile(path, dtype=np.uint8, count=n * fsz)
-        if yuv.size < n * fsz:
-            continue
-        ref_bs, ref_fb, _ = ref_encode(yuv, w, h, n, qp, 30.0)
-        bs, fb = emu_encode(emu, yuv, w, h, n, qp, 30.0)
-        assert fb == ref_fb and bs == bytes(ref_bs), path
-        ran += 1
-    if not ran:
-        pytest.skip("no reference clips on this machine")
+    """more of the reference's own res/*.yuv clips (first pictures; the 1280x720 one as a 160x96 crop)"""
+    for key in ("power_crop_qp30", "vt160_qp24", "static_qp28"):
+        check_reference_clip(emu, key)
 
 
 EDGE = json.load(open(os.path.join(ROOT, "tests", "golden", "encoder_edge.json")))
@@ -156,26 +140,9 @@ def test_emu_cabac_matches_reference_golden(emu, key):
 
 
 def test_emu_cabac_matches_reference_side_by_side(emu):
-    """the same, against the compiled reference on its own clips, both profiles"""
-    if not h264lib.have_ref():
-        pytest.skip("reference build not on this machine")
-    import sys
-    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-    from make_encoder_golden import ref_encode
-    clips = [("/root/reference/res/CiscoVT2people_160x96_6fps.yuv", 160, 96, 5, 24), ("/root/reference/res/Static_152_100.yuv", 152, 100, 8, 28)]
-    ran = 0
-    for path, w, h, n, qp in clips:
-        fsz = w * h * 3 // 2
-        if not os.path.exists(path) or os.path.getsize(path) < n * fsz:
-            continue
-        yuv = np.fromfile(path, dtype=np.uint8, count=n * fsz)
-        for prof in (0, 77):
-            ref_bs, ref_fb, _ = ref_encode(yuv, w, h, n, qp, 30.0, entropy=(1, prof))
-            bs, fb = emu_encode(emu, yuv, w, h, n, qp, 30.0, entropy=(1, prof))
-            assert fb == ref_fb and bs == bytes(ref_bs), (path, prof)
-        ran += 1
-    if not ran:
-        pytest.skip("no reference clips on this machine")
+    """the same, against the reference's bitstreams of its own clips, both profiles"""
+    for key in ("vt160_n5_qp24_cabac0", "vt160_n5_qp24_cabac77", "static_qp28_cabac0", "static_qp28_cabac77"):
+        check_reference_clip(emu, key)
 
 
 @pytest.mark.parametrize("key", sorted(EDGE["intra_period"]))

@@ -11,7 +11,7 @@
 
 #include <vector>
 
-#include "codec_api.h"
+#include "b2h264_wels_abi.h"
 
 typedef long (*create_fn)(ISVCDecoder**);
 typedef void (*destroy_fn)(ISVCDecoder*);

@@ -1,8 +1,8 @@
 // wels_driver.cpp — TEST INFRASTRUCTURE.  An application written against the reference's public API
 // (codec/api/wels/codec_api.h) that loads "some libopenh264" with dlopen and encodes a clip through
-// WelsCreateSVCEncoder / InitializeExt / EncodeFrame.  The tests run the SAME binary once with the compiled
-// reference (oracle/_ref/libopenh264_ref.so) and once with openh264_b200/libopenh264_b200_wels.so and require
-// identical bitstreams and identical SFrameBSInfo layouts: that is the drop-in claim of include/b2h264_wels_api.h.
+// WelsCreateSVCEncoder / InitializeExt / EncodeFrame.  The tests require openh264_b200/libopenh264_b200_wels.so to
+// give the bitstreams and SFrameBSInfo layouts this binary got from the compiled reference (oracle/_ref/libopenh264_ref.so,
+// stored in tests/golden/wels_api.json): that is the drop-in claim of include/b2h264_wels_api.h.
 //   wels_driver <lib.so> <in.yuv> <w> <h> <frames> <qp> <force_idr_at|-1> <out.264> <out.layout>
 #include <dlfcn.h>
 #include <stdio.h>
@@ -11,7 +11,7 @@
 
 #include <vector>
 
-#include "codec_api.h"
+#include "b2h264_wels_abi.h"
 
 typedef int (*create_fn)(ISVCEncoder**);
 typedef void (*destroy_fn)(ISVCEncoder*);

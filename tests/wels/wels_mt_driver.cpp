@@ -19,7 +19,7 @@
 #include <thread>
 #include <vector>
 
-#include "codec_api.h"
+#include "b2h264_wels_abi.h"
 
 typedef int (*create_fn)(ISVCEncoder**);
 typedef void (*destroy_fn)(ISVCEncoder*);
